@@ -3,6 +3,7 @@
 bench.py -- anomaly windows/sec of gordo's per-machine autoencoder anomaly path on N B200s.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config c2|c3|c4|c5]
+                  [--dump-outputs DIR]
 
 Workloads (BASELINE.json `configs`; SURVEY.md §8d fixes the synthetic inputs: Machine m draws from
 default_rng(20260921 + m)):
@@ -85,6 +86,38 @@ def machine_thresholds(rng, T):
 def c3_machine_shape(m, cfg):
     """SURVEY.md §8d: T_m = 20 + (m*37 mod 81); every 4th Machine is an LSTM autoencoder (lookback 16)."""
     return 20 + (m * 37) % 81, (m % 4 == 3)
+
+
+DUMP_BYTES = 60 << 20     # --dump-outputs: at most this many bytes of array data (+ one .npy header per array)
+DUMP_SEED = 0
+
+
+def dump_outputs(dump_dir, columns):
+    """
+    --dump-outputs: write the output arrays of the timed path's last step as DIR/<name>.npy (float32 / float64).
+    When they hold more than DUMP_BYTES (counted at 8 bytes a value), they must share their first axis (rows), and
+    the same fixed, seeded sample of rows (sorted, default_rng(DUMP_SEED)) is taken from every one of them, so two
+    builds of the project can be compared array by array.
+    """
+    import torch
+    os.makedirs(dump_dir, exist_ok=True)
+    shapes = [tuple(t.shape) for t in columns.values()]
+    rows = shapes[0][0]
+    idx = None
+    if sum(8 * int(np.prod(s, dtype=np.int64)) for s in shapes) > DUMP_BYTES:
+        if any(s[0] != rows for s in shapes):
+            raise ValueError("dump_outputs: arrays to be sampled must share their first axis")
+        per_row = sum(8 * int(np.prod(s[1:], dtype=np.int64)) for s in shapes)
+        idx = np.sort(np.random.default_rng(DUMP_SEED).choice(rows, size=DUMP_BYTES // per_row, replace=False))
+    for name, t in columns.items():
+        if torch.is_tensor(t):
+            arr = (t if idx is None else t.index_select(0, torch.as_tensor(idx, device=t.device))).detach().cpu().numpy()
+        else:
+            arr = np.asarray(t) if idx is None else np.asarray(t)[idx]
+        arr = arr.astype(np.float64 if arr.dtype == np.float64 else np.float32, copy=False)
+        np.save(os.path.join(dump_dir, f"{name}.npy"), arr)
+    what = f"{rows} rows" if idx is None else f"{len(idx)} of {rows} rows, seed {DUMP_SEED}"
+    print(f"bench: wrote {len(columns)} output arrays ({what}) to {dump_dir}", file=sys.stderr)
 
 
 def ff_bytes_per_window(T, conf=True):
@@ -490,7 +523,7 @@ def build_ff_fleet(ctx, name, machines=None):
     return fleet, Schedule([rows] * M), x_host, x_dev
 
 
-def run_ff(ctx, args, name, steps, warmup, with_cpu=True, with_other=True):
+def run_ff(ctx, args, name, steps, warmup, with_cpu=True, with_other=True, dump_dir=None):
     torch = ctx.torch
     cfg = CONFIGS[name]
     T, rows = cfg["tags"], cfg["rows"]
@@ -504,6 +537,8 @@ def run_ff(ctx, args, name, steps, warmup, with_cpu=True, with_other=True):
         step()
     sampler = ClockSampler(ctx.local); sampler.start()
     ms_step = ctx.timed(step, steps)
+    if dump_dir and ctx.rank == 0:
+        dump_outputs(dump_dir, out)                                 # before the other precisions overwrite `out`
     other = []
     if with_other:
         for oprec in ("f16x3", "bf16", "f32"):
@@ -617,7 +652,7 @@ def lstm_shards(n_machines, rows, L, world):
     return out
 
 
-def run_lstm(ctx, args, name, steps, warmup, with_cpu=True):
+def run_lstm(ctx, args, name, steps, warmup, with_cpu=True, dump_dir=None):
     torch = ctx.torch
     from gordo_b200.fleet import FFFleet, Schedule
     from gordo_b200.lstm import LSTMFleet
@@ -651,13 +686,21 @@ def run_lstm(ctx, args, name, steps, warmup, with_cpu=True):
     y_off = np.concatenate([[0], np.cumsum(counts)])[:-1] + (L - 1)
     n_win = int(sum(w1 - w0 for _, w0, w1 in mine))
 
+    last = {}                                                    # --dump-outputs: the columns of the latest step
+
     def step():
         out, off = fleet.predict(sched, x_dev, max_windows=18944, precision=prec)
-        return out, FFFleet.score_outputs(out, x_dev, off, y_off, err_scale=err_scale)
+        res = FFFleet.score_outputs(out, x_dev, off, y_off, err_scale=err_scale)
+        if dump_dir:
+            last.clear(); last["model-output"] = out; last.update(res)
+        return out, res
     for _ in range(max(1, warmup)):
         step()
     sampler = ClockSampler(ctx.local); sampler.start()
     ms_step = ctx.timed(step, steps)
+    if dump_dir and ctx.rank == 0:
+        dump_outputs(dump_dir, last)
+    last.clear()
     # e2e: pinned host samples in, host columns out
     host_cols = {}
 
@@ -731,7 +774,7 @@ def c3_fleet_machines(ctx, name, machines_per_gpu=None, rows=None):
     return out, shapes, mine
 
 
-def run_build(ctx, args, name, steps, warmup, with_cpu=True):
+def run_build(ctx, args, name, steps, warmup, with_cpu=True, dump_dir=None):
     torch = ctx.torch
     from gordo_b200.builder import FleetBuild
     cfg = CONFIGS[name]
@@ -754,6 +797,11 @@ def run_build(ctx, args, name, steps, warmup, with_cpu=True):
     clocks = sampler.stop()
     (ms_step,) = ctx.max_over_ranks([dt * 1e3])
     (windows,) = ctx.sum_over_ranks([windows_rank])
+    if dump_dir and ctx.rank == 0:
+        # what the callers receive: each fitted detector's thresholds, in the order of this rank's Machines
+        dump_outputs(dump_dir, {
+            "aggregate-threshold": np.array([float(r[0].aggregate_threshold_) for r in res], np.float64),
+            "feature-thresholds": np.concatenate([np.asarray(r[0].feature_thresholds_, np.float64) for r in res])})
     line = None
     if ctx.rank == 0:
         thr = [float(r[0].aggregate_threshold_) for r in res[:4]]
@@ -893,11 +941,11 @@ def run_ours(args):
     kind = CONFIGS[name]["kind"]
     t_start = time.perf_counter()
     if kind == "ff":
-        line = run_ff(ctx, args, name, args.steps, args.warmup)
+        line = run_ff(ctx, args, name, args.steps, args.warmup, dump_dir=args.dump_outputs)
     elif kind == "lstm":
-        line = run_lstm(ctx, args, name, args.steps, args.warmup)
+        line = run_lstm(ctx, args, name, args.steps, args.warmup, dump_dir=args.dump_outputs)
     else:
-        line = run_build(ctx, args, name, args.steps, args.warmup)
+        line = run_build(ctx, args, name, args.steps, args.warmup, dump_dir=args.dump_outputs)
     # the default line also carries the other single-pass configurations, measured the same way in the same job.
     # Collective-free (see Ctx.collective): each rank measures its shard alone, one all_gather combines them.
     extras = {}
@@ -988,7 +1036,14 @@ def main():
     ap.add_argument("--no-bind", action="store_true", help="do not bind the rank to the GPU's NUMA node")
     ap.add_argument("--no-extras", action="store_true", help="default run: skip the c5 / c4 side measurements")
     ap.add_argument("--extras-budget", type=float, default=150.0, help="seconds after which extras are skipped")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the output columns of the last step (rank 0's Machines; a fixed, "
+                         "seeded sample of rows when larger than 60 MB) as DIR/<column>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     if args.impl == "ours" and args.warmup < 3:
         args.warmup = 3
     if args.config == "c3" and args.steps > 2 and "--steps" not in " ".join(sys.argv):

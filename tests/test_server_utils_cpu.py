@@ -1,13 +1,12 @@
 """
-§8 f-4 wire formats (CPU): gordo_b200.server.utils against the reference's own gordo/server/utils.py (run from
-/root/reference with flask / werkzeug / gordo-core stubbed, in a subprocess, where the reference exists), and the
+§8 f-4 wire formats (CPU): gordo_b200.server.utils against what the reference's own gordo/server/utils.py produced
+(tests/golden/server_codec_golden.json, recorded by tests/golden/make_server_codec_golden.py), and the
 fleet fast paths (column groups -> parquet bytes / nested dict without the DataFrame pivot) against the frame path.
 """
+import base64
+import io
 import json
 import os
-import subprocess
-import sys
-import textwrap
 
 import numpy as np
 import pandas as pd
@@ -59,36 +58,60 @@ def test_empty_and_plain_frames():
     pd.testing.assert_frame_equal(su.dataframe_from_dict(plain.to_dict()), plain)
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/gordo"), reason="/root/reference is not on this box")
+CODEC_CASES = ("time_index", "no_index")
+
+
+def codec_frame(case):
+    """The anomaly frame of ``_groups()``, with a 10-minute time index or none."""
+    if case == "time_index":
+        index, freq = pd.date_range("2020-03-01", periods=40, freq="10min", tz="UTC"), pd.Timedelta("10min")
+    else:
+        index, freq = None, None
+    return mu.assemble_frame(_groups(), index, freq)
+
+
+def frame_record(df):
+    """A frame as plain JSON data: columns, index, dtypes and every value by column (JSON floats round-trip exactly)."""
+    col = lambda c: list(c) if isinstance(c, tuple) else c
+    cell = lambda v: v if v is None or isinstance(v, (bool, int, float)) else str(v)
+    return {"columns": [col(c) for c in df.columns], "column_type": type(df.columns).__name__,
+            "column_names": list(df.columns.names), "index": [str(v) for v in df.index],
+            "index_type": type(df.index).__name__, "index_dtype": str(df.index.dtype), "index_name": df.index.name,
+            "index_freq": getattr(df.index, "freqstr", None), "dtypes": [str(t) for t in df.dtypes],
+            "values": [[cell(v) for v in df.iloc[:, j].tolist()] for j in range(df.shape[1])]}
+
+
+def _read_parquet_as_gordo_does(raw):
+    import pyarrow.parquet as pq
+    return pq.read_table(io.BytesIO(raw)).to_pandas()
+
+
 def test_codecs_match_the_reference_functions():
-    script = "import sys; sys.path.insert(0, %r)\n" % ROOT + textwrap.dedent("""
-        import importlib.util, json, sys, types
-        import numpy as np, pandas as pd
-        def stub(name, **kw):
-            m = types.ModuleType(name); m.__dict__.update(kw); sys.modules[name] = m; return m
-        stub("flask", request=None, g=None, jsonify=None, make_response=None, Response=object)
-        stub("werkzeug"); stub("werkzeug.exceptions", NotFound=Exception, UnprocessableEntity=Exception, InternalServerError=Exception)
-        g = stub("gordo"); g.__path__ = []; g.serializer = None
-        stub("gordo.serializer")
-        srv = stub("gordo.server"); srv.__path__ = ["/root/reference/gordo/server"]
-        stub("gordo.server.properties", get_tags=None, get_target_tags=None)
-        spec = importlib.util.spec_from_file_location("gordo.server.utils", "/root/reference/gordo/server/utils.py")
-        ref = importlib.util.module_from_spec(spec); sys.modules["gordo.server.utils"] = ref; spec.loader.exec_module(ref)
-        from gordo_b200.server import utils as su
-        from gordo_b200.machine.model import utils as mu
-        from tests.test_server_utils_cpu import _groups
-        for index, freq in ((pd.date_range("2020-03-01", periods=40, freq="10min", tz="UTC"), pd.Timedelta("10min")), (None, None)):
-            groups = _groups()
-            df = mu.assemble_frame(groups, index, freq)
-            # the reference's codec on the frame vs ours on the frame and on the raw column groups
-            assert ref.dataframe_to_dict(df) == su.dataframe_to_dict(df) == su.columns_to_dict(groups, index, freq)
-            want = ref.dataframe_from_parquet_bytes(ref.dataframe_into_parquet_bytes(df))
-            pd.testing.assert_frame_equal(want, ref.dataframe_from_parquet_bytes(su.dataframe_into_parquet_bytes(df)))
-            pd.testing.assert_frame_equal(want, ref.dataframe_from_parquet_bytes(su.columns_into_parquet_bytes(groups, index, freq)))
-            pd.testing.assert_frame_equal(want, su.dataframe_from_parquet_bytes(ref.dataframe_into_parquet_bytes(df)))
-            d = json.loads(json.dumps(ref.dataframe_to_dict(df), default=str))
-            pd.testing.assert_frame_equal(ref.dataframe_from_dict(d), su.dataframe_from_dict(d))
-        print("OK")
-    """)
-    r = subprocess.run([sys.executable, "-c", script], capture_output=True, text=True, timeout=300)
-    assert r.returncode == 0 and "OK" in r.stdout, r.stdout + "\n" + r.stderr
+    """Against the original gordo's own codecs, recorded by tests/golden/make_server_codec_golden.py."""
+    with open(os.path.join(ROOT, "tests", "golden", "server_codec_golden.json")) as f:
+        golden = json.load(f)
+    assert sorted(golden) == sorted(CODEC_CASES)
+    for case in CODEC_CASES:
+        _check_codecs(case, golden[case])
+
+
+def _check_codecs(case, want):
+    import pyarrow.parquet as pq
+    df = codec_frame(case)
+    index, freq = (df.index, pd.Timedelta("10min")) if case == "time_index" else (None, None)
+    groups = _groups()
+    # gordo's JSON body of the frame vs ours on the frame and on the raw column groups
+    d = su.dataframe_to_dict(df)
+    assert d == su.columns_to_dict(groups, index, freq), case
+    assert json.loads(json.dumps(d, default=str)) == want["to_dict"], case
+    # gordo's parquet bytes vs ours: the same Arrow table (schema, pandas metadata, data) ...
+    ref_raw = base64.b64decode(want["parquet_base64"])
+    ref_table = pq.read_table(io.BytesIO(ref_raw))
+    for raw in (su.dataframe_into_parquet_bytes(df), su.columns_into_parquet_bytes(groups, index, freq)):
+        table = pq.read_table(io.BytesIO(raw))
+        assert table.equals(ref_table) and table.schema.metadata == ref_table.schema.metadata, case
+        # ... which gordo's reader turns into the frame it read from its own bytes
+        assert frame_record(_read_parquet_as_gordo_does(raw)) == want["from_parquet"], case
+    # our reader on gordo's bytes, and our dict reader on gordo's JSON body, give the frames gordo's readers gave
+    assert frame_record(su.dataframe_from_parquet_bytes(ref_raw)) == want["from_parquet"], case
+    assert frame_record(su.dataframe_from_dict(want["to_dict"])) == want["from_dict"], case
