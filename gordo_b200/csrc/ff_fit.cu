@@ -17,7 +17,6 @@
 // one feature (forward, backward A) or one weight (backward B), reads activations / deltas as 16-byte
 // words along the batch and a weight once per 4 FMAs; samples past the batch end carry zero deltas.
 #include "common.cuh"
-#include <stdlib.h>
 
 namespace {
 
@@ -342,306 +341,6 @@ ff_fit_kernel(const __grid_constant__ FitArgs a) {
     if (tid == 0 && a.adam_t) a.adam_t[job] = t;
 }
 
-
-// =====================================================================================================================
-// ff_fit_mma_kernel: the same fit, with the three GEMM families of a step on the tensor cores (warp-level
-// mma.sync.m16n8k8 tf32) at fp32 accuracy: every operand is split hi + lo (tf32 each) as it is loaded and
-// A_lo.B_hi + A_hi.B_lo + A_hi.B_hi accumulate in fp32 ("3xTF32": product error < 2^-21).  tcgen05 is the wrong
-// tool here -- a batch-32 step is a dependent chain of 20 tiny GEMMs and a tensor-memory round trip per link costs
-// more than the GEMM -- while mma.sync keeps accumulators in registers: a warp owns one 16x8 output tile,
-//   forward : C[b][n]  = bias[n] + sum_k H_l[k][b]   W[k][n]      A = H (feature-major: conflict-free with Bs = Bp + 8)
-//   deltas  : C[b][i]  = sum_n D_{l+1}[n][b] W[i][n]              then (+ l1 sign(h)) * act'(h)
-//   gradient: G[i][n]  = sum_b H_l[i][b] D_{l+1}[n][b]            K = the batch; Adam runs on the accumulator fragment
-// Same layouts, state placement (W, m, v in shared memory), phases, barriers and arithmetic order of everything else as
-// ff_fit_kernel, which stays as the path for topologies whose state does not fit and as the parity reference
-// (GB200_FF_FIT=simt).
-__device__ __forceinline__ void split_tf32(float x, uint32_t& hi, uint32_t& lo) {
-    asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(hi) : "f"(x));
-    const float r = x - __uint_as_float(hi);
-    asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(lo) : "f"(r));
-}
-__device__ __forceinline__ void mma_tf32(float (&c)[4], const uint32_t (&a)[4], const uint32_t (&b)[2]) {
-    asm volatile("mma.sync.aligned.m16n8k8.row.col.f32.tf32.tf32.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%0,%1,%2,%3};"
-                 : "+f"(c[0]), "+f"(c[1]), "+f"(c[2]), "+f"(c[3])
-                 : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b[0]), "r"(b[1]));
-}
-// one K step of a 16x8 tile: big = A_hi.B_hi, small = A_lo.B_hi + A_hi.B_lo (two independent accumulator chains)
-template <bool ONE>
-__device__ __forceinline__ void mma3(float (&big)[4], float (&small)[4], const float (&af)[4], const float (&bf)[2]) {
-    if (ONE) {                          // diagnostic only (GB200_FF_FIT=mma1): plain TF32, one MMA per K step
-        uint32_t ah[4], bh[2];
-        #pragma unroll
-        for (int i = 0; i < 4; ++i) asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(ah[i]) : "f"(af[i]));
-        #pragma unroll
-        for (int i = 0; i < 2; ++i) asm("cvt.rna.tf32.f32 %0, %1;" : "=r"(bh[i]) : "f"(bf[i]));
-        mma_tf32(big, ah, bh);
-        return;
-    }
-    uint32_t ah[4], al[4], bh[2], bl[2];
-    #pragma unroll
-    for (int i = 0; i < 4; ++i) split_tf32(af[i], ah[i], al[i]);
-    #pragma unroll
-    for (int i = 0; i < 2; ++i) split_tf32(bf[i], bh[i], bl[i]);
-    mma_tf32(small, al, bh);
-    mma_tf32(small, ah, bl);
-    mma_tf32(big, ah, bh);
-}
-
-template <bool ONE>
-__global__ void __launch_bounds__(FIT_THREADS, 1)
-ff_fit_mma_kernel(const __grid_constant__ FitArgs a) {
-    extern __shared__ __align__(16) float smem[];
-    __shared__ float red[FIT_THREADS / 32];
-    __shared__ int s_argmax_hits;
-
-    const int job = a.order ? a.order[blockIdx.x] : blockIdx.x, tid = threadIdx.x;
-    const int warp = tid >> 5, lane = tid & 31, g = lane >> 2, t4 = lane & 3;
-    constexpr int NWARPS = FIT_THREADS / 32;
-    const int L = a.arch.n_layers;
-    const int T_in = a.arch.widths[0], T_out = a.arch.widths[L];
-    const int B = a.batch;
-    const int Bp = a.Bq;                 // here: the batch rounded up to 16 (MMA rows); Bs = Bp + 8
-    const int Bs = a.Bs;
-    const int64_t P = a.n_params;
-
-    float* hbuf = smem;
-    float* Dall = hbuf + a.h_floats;
-    float* W = Dall + a.h_floats;
-    float* Mo = W + P;
-    float* Vo = Mo + P;
-    float* gW = a.params + (size_t)job * P;
-    float* gM = a.adam_mv + (size_t)job * 2 * P;
-    float* gV = gM + P;
-    for (int64_t i = tid; i < P; i += FIT_THREADS) { W[i] = gW[i]; Mo[i] = gM[i]; Vo[i] = gV[i]; }
-
-    const int64_t r_lo = a.lo[job];
-    const int n = (int)(a.hi[job] - r_lo);
-    const int slot = a.scale_slot ? a.scale_slot[job] : job;
-    const float* sc = a.in_scale ? a.in_scale + (size_t)slot * T_in : nullptr;
-    const float* mn = a.in_min ? a.in_min + (size_t)slot * T_in : nullptr;
-    const float* ysrc = a.y ? a.y : a.x;
-    const int32_t* perm = a.perm_pool ? a.perm_pool + a.perm_off[job] : nullptr;
-    int64_t t = a.adam_t ? a.adam_t[job] : 0;
-    const float b1 = a.adam.beta_1, b2 = a.adam.beta_2, eps = a.adam.epsilon, lr = a.adam.lr;
-
-    int hoffs[GB200_MAX_LAYERS + 1]; int poffs[GB200_MAX_LAYERS];
-    {
-        int ho = 0, po = 0;
-        for (int l = 0; l < L; ++l) {
-            hoffs[l] = ho; poffs[l] = po;
-            ho += a.arch.widths[l] * Bs; po += a.arch.widths[l] * a.arch.widths[l + 1] + a.arch.widths[l + 1];
-        }
-        hoffs[L] = ho;
-    }
-    __syncthreads();
-
-    for (int e = 0; e < a.epochs; ++e) {
-        double loss_acc = 0.0; int hits_acc = 0;          // meaningful in thread 0 only
-        for (int s0 = 0; s0 < n; s0 += B) {
-            const int nb = min(B, n - s0);
-            // ---- gather + MinMax scale; samples past the batch end are zero (finite activations, zero deltas)
-            for (int i = tid; i < Bp * T_in; i += FIT_THREADS) {
-                const int b = i / T_in, k = i - b * T_in;
-                float v = 0.0f;
-                if (b < nb) {
-                    const int64_t r = r_lo + (perm ? perm[(int64_t)e * n + s0 + b] : s0 + b);
-                    v = a.x[r * T_in + k];
-                    if (sc) v = fmaf(v, sc[k], mn[k]);
-                }
-                hbuf[k * Bs + b] = v;
-            }
-            if (tid == 0) s_argmax_hits = 0;
-            __syncthreads();
-            // ---- forward
-            float l1_sum = 0.0f;
-            for (int l = 0; l < L; ++l) {
-                const int win = a.arch.widths[l], wout = a.arch.widths[l + 1];
-                const int code = a.arch.acts[l];
-                const float* Wl = W + poffs[l]; const float* bl = Wl + win * wout;
-                const float* hin = hbuf + hoffs[l]; float* hout = hbuf + hoffs[l + 1];
-                const float c1 = a.arch.l1[l];
-                const int MT = Bp >> 4, NT = (wout + 7) >> 3;
-                for (int tile = warp; tile < MT * NT; tile += NWARPS) {
-                    const int mt = tile % MT, nt = tile / MT;
-                    const int m0 = mt << 4, n0 = nt << 3;
-                    const int nB = n0 + g;                       // B-fragment column of this lane
-                    const bool nBv = nB < wout;
-                    const int nc0 = n0 + 2 * t4, nc1 = nc0 + 1;  // C-fragment columns of this lane
-                    float big[4], small[4] = {0.0f, 0.0f, 0.0f, 0.0f};
-                    big[0] = big[2] = nc0 < wout ? bl[nc0] : 0.0f;
-                    big[1] = big[3] = nc1 < wout ? bl[nc1] : 0.0f;
-                    for (int k0 = 0; k0 < win; k0 += 8) {
-                        const int ka = k0 + t4, kb = ka + 4;
-                        const bool kav = ka < win, kbv = kb < win;
-                        float af[4], bf[2];
-                        af[0] = kav ? hin[ka * Bs + m0 + g] : 0.0f;     af[1] = kav ? hin[ka * Bs + m0 + g + 8] : 0.0f;
-                        af[2] = kbv ? hin[kb * Bs + m0 + g] : 0.0f;     af[3] = kbv ? hin[kb * Bs + m0 + g + 8] : 0.0f;
-                        bf[0] = (kav && nBv) ? Wl[ka * wout + nB] : 0.0f;
-                        bf[1] = (kbv && nBv) ? Wl[kb * wout + nB] : 0.0f;
-                        mma3<ONE>(big, small, af, bf);
-                    }
-                    #pragma unroll
-                    for (int q = 0; q < 4; ++q) {
-                        const int nn = (q & 1) ? nc1 : nc0, b = m0 + g + ((q & 2) ? 8 : 0);
-                        if (nn < wout) {
-                            const float o = gb_act(code, big[q] + small[q]);
-                            hout[nn * Bs + b] = o;
-                            if (c1 != 0.0f && b < nb) l1_sum += c1 * fabsf(o);
-                        }
-                    }
-                }
-                __syncthreads();
-            }
-            // ---- loss, dLoss/dz_L, accuracy (as ff_fit_kernel)
-            const float* hL = hbuf + hoffs[L];
-            float* DL = Dall + hoffs[L];
-            float sq = 0.0f;
-            {
-                const float inv = 2.0f / (float)(nb * T_out);
-                const int code = a.arch.acts[L - 1];
-                const float cL = a.arch.l1[L - 1] * (a.l1_mean ? 1.0f / (float)nb : 1.0f);
-                for (int i = tid; i < Bp * T_out; i += FIT_THREADS) {
-                    const int b = i / T_out, nn = i - b * T_out;
-                    float dv = 0.0f;
-                    if (b < nb) {
-                        const int64_t r = r_lo + (perm ? perm[(int64_t)e * n + s0 + b] : s0 + b);
-                        const float yh = hL[nn * Bs + b];
-                        const float diff = yh - ysrc[r * T_out + nn];
-                        sq = fmaf(diff, diff, sq);
-                        float dh = inv * diff;
-                        if (cL != 0.0f) dh += cL * (yh > 0.0f ? 1.0f : (yh < 0.0f ? -1.0f : 0.0f));
-                        dv = dh * act_grad_from_h(code, yh);
-                    }
-                    DL[nn * Bs + b] = dv;
-                }
-                if (a.hist_acc) {
-                    for (int b = tid; b < nb; b += FIT_THREADS) {
-                        const int64_t r = r_lo + (perm ? perm[(int64_t)e * n + s0 + b] : s0 + b);
-                        int hit;
-                        if (T_out == 1) {
-                            hit = ((hL[b] > 0.5f ? 1.0f : 0.0f) == ysrc[r]) ? 1 : 0;
-                        } else {
-                            int ay = 0, ap = 0; float by = ysrc[r * T_out], bp = hL[b];
-                            for (int j = 1; j < T_out; ++j) {
-                                const float vy = ysrc[r * T_out + j], vp = hL[j * Bs + b];
-                                if (vy > by) { by = vy; ay = j; }
-                                if (vp > bp) { bp = vp; ap = j; }
-                            }
-                            hit = ay == ap;
-                        }
-                        if (hit) atomicAdd(&s_argmax_hits, 1);
-                    }
-                }
-            }
-            if (a.hist_loss) {
-                const float tot_sq = block_sum(sq, red);
-                const float tot_l1 = block_sum(l1_sum, red);
-                if (tid == 0) {
-                    const float batch_loss = tot_sq / (float)(nb * T_out) + (a.l1_mean ? tot_l1 / (float)nb : tot_l1);
-                    loss_acc += (double)batch_loss * nb;
-                    hits_acc += s_argmax_hits;
-                }
-            } else {
-                __syncthreads();
-            }
-            t += 1;
-            const float tf = (float)t;
-            const float alpha = lr * sqrtf(1.0f - powf(b2, tf)) / (1.0f - powf(b1, tf));
-            const float l1_scale = a.l1_mean ? 1.0f / (float)nb : 1.0f;
-            // ---- deltas, l = L-1 .. 1:  D_l[i][b] = (sum_n D_{l+1}[n][b] W_l[i][n] + l1 sign(h)) act'(h)
-            for (int l = L - 1; l >= 1; --l) {
-                const int win = a.arch.widths[l], wout = a.arch.widths[l + 1];
-                const float* Wl = W + poffs[l];
-                const float* hin = hbuf + hoffs[l];
-                const float* Dcur = Dall + hoffs[l + 1];
-                float* Dnext = Dall + hoffs[l];
-                const int pcode = a.arch.acts[l - 1];
-                const float c1 = a.arch.l1[l - 1] * l1_scale;
-                const int MT = Bp >> 4, NT = (win + 7) >> 3;
-                for (int tile = warp; tile < MT * NT; tile += NWARPS) {
-                    const int mt = tile % MT, it = tile / MT;
-                    const int m0 = mt << 4, i0 = it << 3;
-                    const int iB = i0 + g;                        // B-fragment column (output feature) of this lane
-                    const bool iBv = iB < win;
-                    float big[4] = {0.0f, 0.0f, 0.0f, 0.0f}, small[4] = {0.0f, 0.0f, 0.0f, 0.0f};
-                    for (int j0 = 0; j0 < wout; j0 += 8) {
-                        const int ja = j0 + t4, jb = ja + 4;
-                        const bool jav = ja < wout, jbv = jb < wout;
-                        float af[4], bf[2];
-                        af[0] = jav ? Dcur[ja * Bs + m0 + g] : 0.0f;    af[1] = jav ? Dcur[ja * Bs + m0 + g + 8] : 0.0f;
-                        af[2] = jbv ? Dcur[jb * Bs + m0 + g] : 0.0f;    af[3] = jbv ? Dcur[jb * Bs + m0 + g + 8] : 0.0f;
-                        bf[0] = (jav && iBv) ? Wl[iB * wout + ja] : 0.0f;
-                        bf[1] = (jbv && iBv) ? Wl[iB * wout + jb] : 0.0f;
-                        mma3<ONE>(big, small, af, bf);
-                    }
-                    #pragma unroll
-                    for (int q = 0; q < 4; ++q) {
-                        const int i = i0 + 2 * t4 + (q & 1), b = m0 + g + ((q & 2) ? 8 : 0);
-                        if (i < win) {
-                            const float hv = hin[i * Bs + b];
-                            float acc = big[q] + small[q];
-                            if (c1 != 0.0f) acc += c1 * (hv > 0.0f ? 1.0f : (hv < 0.0f ? -1.0f : 0.0f));
-                            Dnext[i * Bs + b] = b < nb ? acc * act_grad_from_h(pcode, hv) : 0.0f;
-                        }
-                    }
-                }
-                __syncthreads();
-            }
-            // ---- gradients + Adam, every layer, no barrier in between: G[i][n] = sum_b H_l[i][b] D_{l+1}[n][b]
-            for (int l = 0; l < L; ++l) {
-                const int win = a.arch.widths[l], wout = a.arch.widths[l + 1];
-                float* Wl = W + poffs[l];
-                const float* hin = hbuf + hoffs[l];
-                const float* Dcur = Dall + hoffs[l + 1];
-                const int n_w = win * wout;
-                auto adam_update = [&](int i, float gr) {
-                    const int p = poffs[l] + i;
-                    float m = Mo[p], v = Vo[p];
-                    m += (gr - m) * (1.0f - b1);
-                    v += (gr * gr - v) * (1.0f - b2);
-                    Mo[p] = m; Vo[p] = v;
-                    Wl[i] -= alpha * m / (sqrtf(v) + eps);
-                };
-                const int MT = (win + 15) >> 4, NT = (wout + 7) >> 3;
-                for (int tile = warp; tile < MT * NT; tile += NWARPS) {
-                    const int mt = tile % MT, nt = tile / MT;
-                    const int i0 = mt << 4, n0 = nt << 3;
-                    const int ia = i0 + g, ib = ia + 8, nB = n0 + g;
-                    const bool iav = ia < win, ibv = ib < win, nBv = nB < wout;
-                    float big[4] = {0.0f, 0.0f, 0.0f, 0.0f}, small[4] = {0.0f, 0.0f, 0.0f, 0.0f};
-                    for (int b0 = 0; b0 < Bp; b0 += 8) {
-                        float af[4], bf[2];
-                        af[0] = iav ? hin[ia * Bs + b0 + t4] : 0.0f;        af[1] = ibv ? hin[ib * Bs + b0 + t4] : 0.0f;
-                        af[2] = iav ? hin[ia * Bs + b0 + t4 + 4] : 0.0f;    af[3] = ibv ? hin[ib * Bs + b0 + t4 + 4] : 0.0f;
-                        bf[0] = nBv ? Dcur[nB * Bs + b0 + t4] : 0.0f;
-                        bf[1] = nBv ? Dcur[nB * Bs + b0 + t4 + 4] : 0.0f;
-                        mma3<ONE>(big, small, af, bf);
-                    }
-                    #pragma unroll
-                    for (int q = 0; q < 4; ++q) {
-                        const int i = (q & 2) ? ib : ia, nn = n0 + 2 * t4 + (q & 1);
-                        if (i < win && nn < wout) adam_update(i * wout + nn, big[q] + small[q]);
-                    }
-                }
-                for (int nn = tid; nn < wout; nn += FIT_THREADS) {
-                    const float* dp = Dcur + nn * Bs;
-                    float gr = 0.0f;
-                    for (int b = 0; b < Bp; ++b) gr += dp[b];
-                    adam_update(n_w + nn, gr);
-                }
-            }
-            __syncthreads();
-        }
-        if (tid == 0) {
-            if (a.hist_loss) a.hist_loss[(size_t)job * a.epochs + e] = n > 0 ? (float)(loss_acc / n) : NAN;
-            if (a.hist_acc) a.hist_acc[(size_t)job * a.epochs + e] = n > 0 ? (float)hits_acc / (float)n : NAN;
-        }
-    }
-    __syncthreads();
-    for (int64_t i = tid; i < P; i += FIT_THREADS) { gW[i] = W[i]; gM[i] = Mo[i]; gV[i] = Vo[i]; }
-    if (tid == 0 && a.adam_t) a.adam_t[job] = t;
-}
-
 }  // namespace
 
 int gb_launch_ff_fit(const gb200_ff_arch* arch, const gb200_adam* adam, int n_jobs,
@@ -671,27 +370,6 @@ int gb_launch_ff_fit(const gb200_ff_arch* arch, const gb200_adam* adam, int n_jo
         fit_order_kernel<<<(n_jobs + 127) / 128, 128, 0, stream>>>(n_jobs, lo, hi, order);
     }
     a.order = order;
-    // ---- tensor-core path (warp-level mma, 3xTF32): when W + both Adam moments + the batch's activations and
-    // deltas (batch rounded up to 16 rows) fit in shared memory.  GB200_FF_FIT=simt forces the CUDA-core kernel.
-    {
-        // Default: the CUDA-core kernel.  The tensor-core version is correct (same parity tests) but measured SLOWER on
-        // the c2 build (512 fits: 383 ms vs 268 ms, profiles/README.md r2f): GB200_FF_FIT=mma selects it.
-        bool want_mma = false, one = false;
-        if (const char* e = getenv("GB200_FF_FIT")) { want_mma = e[0] == 'm'; one = want_mma && e[1] == 'm' && e[2] == 'a' && e[3] == '1'; }
-        const int Bp = (batch_size + 15) / 16 * 16, Bsm = Bp + 8;
-        const size_t need = (2 * (size_t)sum_w * Bsm + 3 * (size_t)a.n_params) * sizeof(float);
-        if (want_mma && need <= cap) {
-            FitArgs m = a;
-            m.Bq = Bp; m.Bs = Bsm; m.h_floats = sum_w * Bsm; m.state_in_smem = 2;
-            auto* mk = one ? ff_fit_mma_kernel<true> : ff_fit_mma_kernel<false>;
-            GB_CUDA_CHECK(gb_allow_max_smem(mk));
-            mk<<<n_jobs, FIT_THREADS, need, stream>>>(m);
-            cudaError_t le = cudaGetLastError();
-            if (order) cudaFreeAsync(order, stream);
-            GB_CUDA_CHECK(le);
-            return GB_OK;
-        }
-    }
     size_t base = 2 * (size_t)a.h_floats * sizeof(float);      // activations + one delta slot per activation
     const bool hg = base > cap;         // the batch's activations go to a global scratch (see the HG note)
     float* scratch = nullptr;

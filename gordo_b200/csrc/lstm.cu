@@ -1082,8 +1082,8 @@ __global__ void lstm_adam_kernel(const __grid_constant__ AdamArgs a) {
     }
 }
 // Last kernel of an optimizer step.  `advance` > 0 moves every group's window cursor (first sample row, windows
-// left) forward by one batch ON THE DEVICE: a step's launches then take identical arguments from one step to
-// the next, which is what lets the whole step be replayed as one CUDA graph.
+// left) forward by one batch on the device.  The kernels of a step read their batch from that cursor, so a group
+// whose windows have run out sees nb = 0 and takes no step: no loss, no Adam update, no step count.
 __global__ void lstm_step_end_kernel(GroupCtx g, int n_groups, int64_t* tcount, const float* loss_sum,
                                      float* epoch_acc, int T_out, float* primer_loss, int advance,
                                      int64_t* rows_cur, int32_t* nwin_cur) {
@@ -1506,45 +1506,17 @@ int gb200_lstm_fit(const gb200_lstm_arch* arch, const gb200_adam* adam, int32_t 
     rc = run_step(1, primer_loss ? primer_loss : d_epoch + 0 /*unused sink*/, 0);
     if (rc) return rc;
     if (!primer_loss) GB_CUDA_CHECK(cudaMemsetAsync(d_epoch, 0, sizeof(float) * J, stream));
-    // (2) main fit: time-ordered batches, shuffle=False (models.py:599-615).  A step is 50-100 small dependent
-    // launches with identical arguments from step to step (the batch position lives on the device), so it can be
-    // replayed as ONE CUDA graph per step: GB200_LSTM_GRAPH=1.  Off by default -- on the c3 build (many concurrent
-    // streams, steps bound by the cluster recurrence kernels, not by launches) the replay measured slower than
-    // stream launches (profiles/README.md r2c); a legacy-default-stream caller cannot capture at all.
+    // (2) main fit: time-ordered batches, shuffle=False (models.py:599-615).  Every job runs the same number of steps,
+    // enough for the job with the most windows; the device cursor stops the others once their windows run out.
     const int n_steps = (max_win + B - 1) / B;
-    cudaGraphExec_t exec = nullptr;
-    bool use_graph = false;
-    { const char* e = getenv("GB200_LSTM_GRAPH"); if (e && atoi(e) == 1 && n_steps >= 4) use_graph = true; }
-    if (use_graph) {
-        cudaGraph_t graph = nullptr;
-        if (cudaStreamBeginCapture(stream, cudaStreamCaptureModeRelaxed) == cudaSuccess) {
-            const int crc = run_step(B, nullptr, B);
-            const cudaError_t ee = cudaStreamEndCapture(stream, &graph);
-            if (crc != GB_OK || ee != cudaSuccess || graph == nullptr ||
-                cudaGraphInstantiate(&exec, graph, 0) != cudaSuccess) exec = nullptr;
-            if (graph) cudaGraphDestroy(graph);
-        }
-        (void)cudaGetLastError();               // a failed capture leaves a sticky-free error behind: clear it
-    }
     for (int e = 0; e < epochs; ++e) {
-        rc = rewind(); if (rc) { if (exec) cudaGraphExecDestroy(exec); return rc; }
+        rc = rewind(); if (rc) return rc;
         for (int s = 0; s < n_steps; ++s) {
-            if (exec) {
-                const cudaError_t le = cudaGraphLaunch(exec, stream);
-                if (le != cudaSuccess) { cudaGraphExecDestroy(exec); gb_set_error("lstm fit: graph launch: %s", cudaGetErrorString(le)); return GB_ERR_CUDA; }
-            } else {
-                rc = run_step(B, nullptr, B);
-                if (rc) return rc;
-            }
+            rc = run_step(B, nullptr, B);
+            if (rc) return rc;
         }
         if (hist_loss) lstm_epoch_end_kernel<<<cdiv(J, 128), 128, 0, stream>>>(J, d_nwin, d_epoch, hist_loss, epochs, e);
         else GB_CUDA_CHECK(cudaMemsetAsync(d_epoch, 0, sizeof(float) * J, stream));
-    }
-    if (exec) {
-        // the executable graph must outlive its last launch: wait for the stream, then release it
-        const cudaError_t se = cudaStreamSynchronize(stream);
-        cudaGraphExecDestroy(exec);
-        if (se != cudaSuccess) { gb_set_error("lstm fit: %s", cudaGetErrorString(se)); return GB_ERR_CUDA; }
     }
     GB_CUDA_CHECK(cudaGetLastError());
     return GB_OK;

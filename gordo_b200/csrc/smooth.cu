@@ -10,15 +10,13 @@
 // the run after warming up on the w-1 rows in front of it; threads of a warp sit on adjacent columns,
 // so a row step of a warp is one contiguous read and one contiguous write.  The moving median keeps
 // the window as a ring of integer keys in shared memory and tracks the rank-k element with one uniform
-// pass per output (smm_rank_kernel below; the round-1 sorted-window version stays selectable with
-// GB200_SMM=legacy).  Mean / EWMA carry their state in float64 registers, in the recurrences pandas
-// uses.  NaN and +-inf are missing values for all three, as pandas' `_prep_values` makes them.
-// Quantile: coalesced whole-row reads, 4 x 8-bit radix select passes over global histograms (further down;
-// the round-1 one-CTA-per-8-columns kernel stays selectable with GB200_QUANTILE=legacy).
+// pass per output (smm_rank_kernel).  Mean / EWMA (smooth_kernel) carry their state in float64 registers,
+// in the recurrences pandas uses.  NaN and +-inf are missing values for all three, as pandas'
+// `_prep_values` makes them.
+// Quantile: coalesced whole-row reads, 4 x 8-bit radix select passes over global histograms (further down).
 #include "common.cuh"
 #include <math.h>
 #include <stdlib.h>
-#include <string.h>
 
 namespace {
 
@@ -31,55 +29,7 @@ struct SmoothArgs {
     double alpha;       // EWMA: 2 / (span + 1)
 };
 
-// sorted window of thread `tid`: element i lives at s[i * nt + tid]
-struct SortedWin {
-    float* s; int nt; int n;
-    __device__ __forceinline__ float& at(int i) { return s[i * nt]; }
-    __device__ __forceinline__ int lower_bound(float x) {        // first i with s[i] >= x
-        int lo = 0, hi = n;
-        while (lo < hi) { const int mid = (lo + hi) >> 1; if (at(mid) < x) lo = mid + 1; else hi = mid; }
-        return lo;
-    }
-    __device__ __forceinline__ void insert(float x) {
-        int i = n;
-        while (i > 0 && at(i - 1) > x) { at(i) = at(i - 1); --i; }
-        at(i) = x; ++n;
-    }
-    __device__ __forceinline__ void remove(float x) {
-        int i = lower_bound(x);
-        for (; i + 1 < n; ++i) at(i) = at(i + 1);
-        --n;
-    }
-    // The outgoing value's slot is refilled by shifting the run between it and the incoming value's
-    // position by one.  Both ends come from binary searches, so the shift loop has a known trip count
-    // and its loads do not depend on its stores (4 independent load/store pairs in flight).
-    __device__ __forceinline__ void replace(float x_old, float x_new) {
-        const int p = lower_bound(x_old);                      // slot of the outgoing value
-        if (x_new >= x_old) {
-            int q = lower_bound(x_new) - 1;                    // last slot holding a value < x_new
-            if (q < p) q = p;
-            int i = p;
-            for (; i + 4 <= q; i += 4) {
-                const float a = at(i + 1), b = at(i + 2), c = at(i + 3), d = at(i + 4);
-                at(i) = a; at(i + 1) = b; at(i + 2) = c; at(i + 3) = d;
-            }
-            for (; i < q; ++i) at(i) = at(i + 1);
-            at(q) = x_new;
-        } else {
-            const int q = lower_bound(x_new);                  // first slot holding a value >= x_new
-            int i = p;
-            for (; i - 4 >= q; i -= 4) {
-                const float a = at(i - 1), b = at(i - 2), c = at(i - 3), d = at(i - 4);
-                at(i) = a; at(i - 1) = b; at(i - 2) = c; at(i - 3) = d;
-            }
-            for (; i > q; --i) at(i) = at(i - 1);
-            at(q) = x_new;
-        }
-    }
-};
-
 __global__ void smooth_kernel(const __grid_constant__ SmoothArgs a) {
-    extern __shared__ float s_win[];
     const int nt = blockDim.x, tid = threadIdx.x;
     const int job = blockIdx.y;
     const int c0 = blockIdx.z * nt;
@@ -96,30 +46,18 @@ __global__ void smooth_kernel(const __grid_constant__ SmoothArgs a) {
     const float* v = a.v + col;
     float* out = a.out + col;
 
-    if (a.method == GB200_SMOOTH_SMM) {
-        SortedWin sw{s_win + tid, nt, 0};
-        const bool odd = (w & 1) != 0;
-        float nx = v[h0 * C], ox = NAN;                  // the next row's values are loaded one step ahead
+    // Both loops are latency-bound: they load the next row's values one step ahead (the store to `out` may alias `v`,
+    // so the compiler moves no load above it) and stay rolled, which keeps the kernel at 48 registers, 5 CTAs per SM.
+    if (a.method == GB200_SMOOTH_SMA) {
+        double sum = 0.0; int nobs = 0;
+        const double inv_w = 1.0 / (double)w;
+        float nx = v[h0 * C], ox = NAN;                  // the row entering / leaving the window (NaN: none leaves)
+        #pragma unroll 1
         for (int64_t r = h0; r < o1; ++r) {
             const float x_new = nx, x_old = ox;
             if (r + 1 < o1) { nx = v[(r + 1) * C]; ox = (r + 1 - w >= h0) ? v[(r + 1 - w) * C] : NAN; }
-            const bool vo = fabsf(x_old) < INFINITY, vn = fabsf(x_new) < INFINITY;   // pandas: NaN and +-inf are missing
-            if (vo && vn) sw.replace(x_old, x_new);
-            else { if (vo) sw.remove(x_old); if (vn) sw.insert(x_new); }
-            if (r >= o0) {
-                float m = NAN;
-                if (sw.n == w)          // w non-NaN observations (min_periods = window)
-                    m = odd ? sw.at(w >> 1) : (float)(0.5 * ((double)sw.at((w >> 1) - 1) + (double)sw.at(w >> 1)));
-                out[r * C] = m;
-            }
-        }
-    } else if (a.method == GB200_SMOOTH_SMA) {
-        double sum = 0.0; int nobs = 0;
-        const double inv_w = 1.0 / (double)w;
-        for (int64_t r = h0; r < o1; ++r) {
-            const float x_new = v[r * C];
             if (fabsf(x_new) < INFINITY) { sum += (double)x_new; ++nobs; }
-            if (r - w >= h0) { const float x_old = v[(r - w) * C]; if (fabsf(x_old) < INFINITY) { sum -= (double)x_old; --nobs; } }
+            if (fabsf(x_old) < INFINITY) { sum -= (double)x_old; --nobs; }
             if (r >= o0) out[r * C] = nobs == w ? (float)(sum * inv_w) : NAN;
         }
     } else {
@@ -133,8 +71,11 @@ __global__ void smooth_kernel(const __grid_constant__ SmoothArgs a) {
         int64_t last = o0 - 1;
         while (last >= j0 && !(fabsf(v[last * C]) < INFINITY)) --last;
         const int64_t e0 = last < j0 ? o0 : max(j0, last - (int64_t)a.halo);
+        float nx = v[e0 * C];
+        #pragma unroll 1
         for (int64_t r = e0; r < o1; ++r) {
-            const float x = v[r * C];
+            const float x = nx;
+            if (r + 1 < o1) nx = v[(r + 1) * C];
             const bool obs = fabsf(x) < INFINITY;
             if (r > e0) {
                 if (avg == avg) {
@@ -150,10 +91,7 @@ __global__ void smooth_kernel(const __grid_constant__ SmoothArgs a) {
     }
 }
 
-// ---------------------------------------------------------------- quantile
-constexpr int Q_THREADS = 256;
-constexpr int Q_BINS = 2048;
-
+// ---------------------------------------------------------------- order-preserving keys of floats
 __device__ __forceinline__ uint32_t f2key(float x) {
     const uint32_t u = __float_as_uint(x);
     return (u & 0x80000000u) ? ~u : (u | 0x80000000u);
@@ -163,10 +101,10 @@ __device__ __forceinline__ float key2f(uint32_t k) {
 }
 
 // ---------------------------------------------------------------- moving median, rank-tracking version
-// The sorted-window kernel above pays two binary searches (dependent shared-memory loads) and a shift whose length
-// differs per lane -- a warp waits for its slowest lane, ~0.85 w moves on white noise -- per output: 87 ms for the
-// c2-sized matrix at w = 144.  This version keeps the window as an UNSORTED ring of order-preserving integer keys and
-// tracks the median itself: when one value leaves and one enters, every rank moves by at most one, so with
+// A sorted window per thread (round 1's kernel) pays two binary searches (dependent shared-memory loads) and a shift
+// whose length differs per lane -- a warp waits for its slowest lane, ~0.85 w moves on white noise -- per output: 87 ms
+// for the c2-sized matrix at w = 144.  This version keeps the window as an UNSORTED ring of order-preserving integer
+// keys and tracks the median itself: when one value leaves and one enters, every rank moves by at most one, so with
 // r = the previous element of rank k (k = w / 2)
 //      new rank-k element   is one of { pred(r), r, succ(r) },
 //      new rank-(k-1) one   is one of { second largest below r, pred(r), r }            (even windows only),
@@ -298,120 +236,6 @@ __global__ void __launch_bounds__(384, 1) smm_rank_kernel(const __grid_constant_
     }
 }
 
-// One CTA = one job x QC adjacent columns: a row's QC values share one or two 32-byte sectors, so the
-// strided column walk costs 1/QC of the L2 traffic of a CTA per column.  Three histogram passes
-// (11 + 11 + 10 bits) select the order statistic of rank k = floor((n-1) q) of every column -- the first
-// pass's histogram also counts the non-NaN rows -- and one more pass finds the next order statistic
-// (count of values <= it, smallest value above it) for the linear interpolation.
-constexpr int QC = 8;
-
-__global__ void __launch_bounds__(Q_THREADS)
-quantile_kernel(const int64_t* __restrict__ lo, const int64_t* __restrict__ hi, const float* __restrict__ v,
-                int C, double q, double* __restrict__ out) {
-    extern __shared__ int qhist[];                    // [QC][Q_BINS]
-    __shared__ uint32_t s_prefix[QC], s_mask[QC], s_mingt[QC];
-    __shared__ long long s_rank[QC], s_n[QC];
-    __shared__ unsigned long long s_le[QC];
-    const int job = blockIdx.y, c0 = blockIdx.x * QC;
-    const int nc = min(QC, C - c0);
-    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-    const int64_t j0 = lo[job], n_rows = hi[job] - j0;
-    const float* base = v + j0 * C + c0;
-    const int shifts[3] = {21, 10, 0}, bits[3] = {11, 11, 10};
-    if (tid < QC) { s_prefix[tid] = 0; s_mask[tid] = 0; s_rank[tid] = 0; s_n[tid] = 0; s_le[tid] = 0; s_mingt[tid] = 0xffffffffu; }
-    for (int p = 0; p < 3; ++p) {
-        const int nb = 1 << bits[p];
-        for (int i = tid; i < QC * Q_BINS; i += Q_THREADS) qhist[i] = 0;
-        __syncthreads();
-        for (int64_t r = tid; r < n_rows; r += Q_THREADS) {
-            const float* row = base + r * C;
-            for (int j = 0; j < nc; ++j) {
-                const float x = row[j];
-                if (x == x) {
-                    const uint32_t k = f2key(x);
-                    if ((k & s_mask[j]) == s_prefix[j]) {
-                        // scores cluster in a few bins (one exponent): when every active lane hits the SAME bin one
-                        // lane adds the count (a shuffle + a vote; MATCH.ANY per element was the kernel's bottleneck),
-                        // otherwise the lanes are spread and plain shared-memory atomics rarely collide
-                        const int bin = (int)((k >> shifts[p]) & (nb - 1));
-                        const unsigned act = __activemask();
-                        const int leader = __ffs(act) - 1;
-                        const int lead_bin = __shfl_sync(act, bin, leader);
-                        if (__all_sync(act, bin == lead_bin)) {
-                            if (lane == leader) atomicAdd(&qhist[j * Q_BINS + bin], __popc(act));
-                        } else {
-                            atomicAdd(&qhist[j * Q_BINS + bin], 1);
-                        }
-                    }
-                }
-            }
-        }
-        __syncthreads();
-        if (warp < nc) {
-            // warp `warp` resolves column `warp`: lane l owns nb/32 consecutive bins
-            const int j = warp, per = nb / 32;
-            const int* h = qhist + j * Q_BINS + lane * per;
-            long long local = 0;
-            for (int i = 0; i < per; ++i) local += h[i];
-            long long incl = local;
-            for (int o = 1; o < 32; o <<= 1) { const long long t = __shfl_up_sync(0xffffffffu, incl, o); if (lane >= o) incl += t; }
-            const long long total = __shfl_sync(0xffffffffu, incl, 31);
-            long long rank = s_rank[j];
-            if (p == 0) { rank = total > 0 ? (long long)floor((double)(total - 1) * q) : 0; if (lane == 0) s_n[j] = total; }
-            const long long before = incl - local;
-            if (total > 0 && rank >= before && rank < before + local) {
-                long long acc = before; int b = 0;
-                for (;; ++b) { const int hb = h[b]; if (rank < acc + hb) break; acc += hb; }
-                s_prefix[j] |= (uint32_t)(lane * per + b) << shifts[p];
-                s_rank[j] = rank - acc;
-            }
-            if (lane == 0) s_mask[j] |= (uint32_t)(nb - 1) << shifts[p];
-        }
-        __syncthreads();
-    }
-    // ---- the next order statistic: #values <= a and the smallest value above a (key order = value order)
-    {
-        unsigned long long le[QC]; uint32_t mg[QC];
-        #pragma unroll
-        for (int j = 0; j < QC; ++j) { le[j] = 0; mg[j] = 0xffffffffu; }
-        for (int64_t r = tid; r < n_rows; r += Q_THREADS) {
-            const float* row = base + r * C;
-            #pragma unroll
-            for (int j = 0; j < QC; ++j) {
-                if (j >= nc) break;
-                const float x = row[j];
-                if (x == x) {
-                    const uint32_t k = f2key(x);
-                    if (k <= s_prefix[j]) ++le[j]; else mg[j] = min(mg[j], k);
-                }
-            }
-        }
-        #pragma unroll
-        for (int j = 0; j < QC; ++j) {
-            for (int o = 16; o > 0; o >>= 1) {
-                le[j] += __shfl_down_sync(0xffffffffu, le[j], o);
-                mg[j] = min(mg[j], __shfl_down_sync(0xffffffffu, mg[j], o));
-            }
-            if (lane == 0 && j < nc) { atomicAdd(&s_le[j], le[j]); atomicMin(&s_mingt[j], mg[j]); }
-        }
-    }
-    __syncthreads();
-    if (tid < nc) {
-        const long long n = s_n[tid];
-        double res = NAN;
-        if (n > 0) {
-            const double h = (double)(n - 1) * q;
-            const long long k = (long long)floor(h);
-            const double frac = h - (double)k;
-            const double va = (double)key2f(s_prefix[tid]);
-            double vb = va;
-            if (frac > 0.0 && k + 1 < n && s_le[tid] < (unsigned long long)(k + 2)) vb = (double)key2f(s_mingt[tid]);
-            res = va + (vb - va) * frac;
-        }
-        out[(size_t)job * C + c0 + tid] = res;
-    }
-}
-
 int max_rows_host(int n_jobs, const int64_t* lo, const int64_t* hi, cudaStream_t stream, int64_t* out) {
     int64_t* h = (int64_t*)malloc(sizeof(int64_t) * 2 * n_jobs);
     if (!h) { gb_set_error("out of host memory"); return GB_ERR_ARG; }
@@ -441,10 +265,9 @@ int gb_launch_smooth(int n_jobs, const int64_t* lo, const int64_t* hi, const flo
     SmoothArgs a{};
     a.lo = lo; a.hi = hi; a.v = v; a.out = out; a.C = n_cols; a.window = window; a.method = method;
     int nt = 256;
-    size_t smem = 0;
-    static const bool legacy_smm = [] { const char* e = getenv("GB200_SMM"); return e && !strcmp(e, "legacy"); }();
-    const bool rank_smm = method == GB200_SMOOTH_SMM && !legacy_smm;
-    if (rank_smm) {
+    size_t smem = 0;                // moving median only
+    const bool smm = method == GB200_SMOOTH_SMM;
+    if (smm) {
         // ring of ceil(w / 4) key quads per thread; as many threads as the shared memory of one SM holds
         const size_t per_thread = (size_t)((window + 3) / 4) * sizeof(uint4);
         nt = 384;
@@ -452,14 +275,6 @@ int gb_launch_smooth(int n_jobs, const int64_t* lo, const int64_t* hi, const flo
         GB_REQUIRE((size_t)nt * per_thread <= GB_SMEM_OPTIN_MAX, "smooth: moving-median window %d too long (max %d)",
                    window, (int)(GB_SMEM_OPTIN_MAX / (32 * sizeof(uint4)) * 4));
         smem = (size_t)nt * per_thread;
-        a.halo = window - 1;
-    } else if (method == GB200_SMOOTH_SMM) {
-        // the sorted windows of a block live in shared memory: fewer threads for long windows
-        const size_t cap = 200 * 1024;
-        while (nt > 32 && (size_t)nt * window * sizeof(float) > cap) nt >>= 1;
-        GB_REQUIRE((size_t)nt * window * sizeof(float) <= cap, "smooth: moving-median window %d too long (max %d)",
-                   window, (int)(cap / (32 * sizeof(float))));
-        smem = (size_t)nt * window * sizeof(float);
         a.halo = window - 1;
     } else if (method == GB200_SMOOTH_SMA) {
         a.halo = window - 1;
@@ -474,7 +289,7 @@ int gb_launch_smooth(int n_jobs, const int64_t* lo, const int64_t* hi, const flo
     int S = a.halo > 512 ? a.halo : 512;
     const int Cc = n_cols < nt ? n_cols : nt;
     const int nsub = nt / Cc;
-    if (rank_smm) {
+    if (smm) {
         // one CTA per SM and a per-run overhead of halo + ~w/2 selection passes: pick the number of CTAs per job
         // (j = 1, 2, ...; S = the rows that leaves per thread) that minimises waves x (S + overhead).  With S fixed
         // at 2048 the c2-sized matrix made 896 CTAs = 6.05 waves of 148.
@@ -493,7 +308,7 @@ int gb_launch_smooth(int n_jobs, const int64_t* lo, const int64_t* hi, const flo
     a.S = S;
     const int64_t rows_per_block = (int64_t)nsub * S;
     dim3 grid((unsigned)((max_rows + rows_per_block - 1) / rows_per_block), n_jobs, (n_cols + nt - 1) / nt);
-    if (rank_smm) {
+    if (smm) {
         auto launch = [&](auto kern) -> int {
             if (smem > 48 * 1024) GB_CUDA_CHECK(gb_allow_max_smem(kern));
             kern<<<grid, nt, smem, stream>>>(a);
@@ -502,9 +317,7 @@ int gb_launch_smooth(int n_jobs, const int64_t* lo, const int64_t* hi, const flo
         };
         return (window & 1) ? launch(smm_rank_kernel<false>) : launch(smm_rank_kernel<true>);
     }
-    if (smem > 48 * 1024)
-        GB_CUDA_CHECK(gb_allow_max_smem(smooth_kernel));
-    smooth_kernel<<<grid, nt, smem, stream>>>(a);
+    smooth_kernel<<<grid, nt, 0, stream>>>(a);
     GB_CUDA_CHECK(cudaGetLastError());
     return GB_OK;
 }
@@ -512,7 +325,7 @@ int gb_launch_smooth(int n_jobs, const int64_t* lo, const int64_t* hi, const flo
 
 namespace {
 // ---------------------------------------------------------------- quantile, coalesced multi-CTA version
-// The one-CTA-per-(job, 8 columns) kernel above walks its columns with a 200-byte stride: every warp load touches 32
+// A CTA per (job, 8 columns) (round 1's kernel) walks its columns with a 200-byte stride: every warp load touches 32
 // sectors, and the load unit's wavefronts -- not the histogram atomics -- bound it (32 ms for the 2.56 GB c2-sized
 // matrix, unchanged when MATCH.ANY was removed).  Here a CTA reads whole rows: thread = (row lane, column) with the
 // column FIXED per thread, so a warp's 32 lanes are 32 adjacent floats of the row-major matrix (fully coalesced), a
@@ -635,16 +448,6 @@ int gb_launch_quantile(int n_jobs, const int64_t* lo, const int64_t* hi, const f
                        double q, double* out, cudaStream_t stream) {
     if (n_jobs <= 0) return GB_OK;
     GB_REQUIRE(q >= 0.0 && q <= 1.0, "quantile: q must be in [0, 1]");
-    bool legacy = false;
-    if (const char* e = getenv("GB200_QUANTILE")) legacy = e[0] == 'l';       // "legacy": the one-CTA-per-8-columns kernel
-    if (legacy) {
-        dim3 grid((n_cols + QC - 1) / QC, n_jobs);
-        const int smem = QC * Q_BINS * (int)sizeof(int);
-        GB_CUDA_CHECK(cudaFuncSetAttribute(quantile_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-        quantile_kernel<<<grid, Q_THREADS, smem, stream>>>(lo, hi, v, n_cols, q, out);
-        GB_CUDA_CHECK(cudaGetLastError());
-        return GB_OK;
-    }
     const int n_items = n_jobs * n_cols;
     const int colchunks = (n_cols + QH_MAXC - 1) / QH_MAXC;
     // rows of a job are split over gx CTAs so that the launch has a few CTAs per SM without knowing the row counts

@@ -373,33 +373,6 @@ def test_estimator_and_detector_with_f16x3_precision():
         np.testing.assert_allclose(frames["f16x3"][col].to_numpy(), frames["f32"][col].to_numpy(), rtol=2e-4, atol=3e-5, err_msg=col)
 
 
-# ----------------------------------------------------------------------------- the tensor-core training kernel (opt-in) stays covered
-@pytest.mark.parametrize("T,batch", [(10, 32), (50, 32), (9, 33)])
-def test_ff_fit_tensor_core_variant_matches_the_default_kernel(T, batch, monkeypatch):
-    """GB200_FF_FIT=mma = ff_fit_mma_kernel (warp-level mma.sync, 3xTF32: fp32-grade); default = the CUDA-core kernel
-    (measured faster): same trajectories."""
-    from gordo_b200.fleet import FFFleet, FFTopology
-    rng = np.random.default_rng(40 + T)
-    spec = factories.feedforward_hourglass(T)
-    topo = FFTopology(spec["widths"], spec["acts"], spec["l1"])
-    fl = FFFleet(topo, 1, DEV)
-    rows = [300, 77]
-    X = torch.from_numpy(rng.random((sum(rows), T)).astype(np.float32)).to(DEV)
-    lo = _i64([0, rows[0]]); hi = _i64([rows[0], sum(rows)])
-    init = torch.from_numpy(np.stack([dense.ff_flatten(dense.ff_init(spec, rng)) for _ in rows])).to(DEV)
-    res = {}
-    for mode in ("mma", "simt"):
-        monkeypatch.setenv("GB200_FF_FIT", mode)
-        p = init.clone()
-        hl, ha, mv, t = fl.fit_jobs(X, None, lo, hi, p, epochs=2, batch_size=batch)
-        torch.cuda.synchronize()
-        res[mode] = (p.cpu().numpy(), hl.cpu().numpy(), ha.cpu().numpy(), mv.cpu().numpy())
-    np.testing.assert_allclose(res["mma"][0], res["simt"][0], rtol=0, atol=2e-4)
-    np.testing.assert_allclose(res["mma"][1], res["simt"][1], rtol=2e-4)
-    np.testing.assert_allclose(res["mma"][2], res["simt"][2], atol=2.0 / min(rows))
-    assert float(np.abs(res["mma"][0] - init.cpu().numpy()).max()) > 1e-3
-
-
 def test_anomaly_response_bodies_equal_the_frame_codecs():
     """model.anomaly_response (column groups -> parquet bytes / JSON dict) == the server codecs applied to model.anomaly's
     frame (gordo/server/blueprints/anomaly.py:57-72), incl. the smooth-* columns the view drops by default."""
